@@ -2,7 +2,7 @@
 """Headline benchmark (BASELINE.json): samples/sec of the 2-layer-1024 LSTM, seq_len 128, batch 256 per GPU, bf16,
 per-step gradient allreduce, synthetic sequences / random-init weights.
 
-    python bench.py --gpus N --steps K --warmup W [--impl ours|reference|baseline]
+    python bench.py --gpus N --steps K --warmup W [--impl ours|reference|baseline] [--dump-outputs DIR]
 
 N > 1 is launched by the driver under torchrun (RANK / LOCAL_RANK / WORLD_SIZE / MASTER_* from the env), one rank
 per GPU.  Rank 0 prints ONE JSON line.  ``value`` is the whole-job aggregate (sum over GPUs); timing is CUDA events
@@ -53,7 +53,32 @@ def parse():
     ap.add_argument("--config", type=int, default=3, choices=[3, 4],
                     help="BASELINE.json config: 3 = 2x1024 T=128 B=256 per-step grad allreduce (headline); "
                          "4 = 4x2048 T=512 B=64 per-epoch parameter average (one average inside the timed region)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="ours: after the device-timed steps, write the loss of the last step and the model variables it left as "
+                         "DIR/<name>.npy (see dump_outputs), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Write ``arrays`` (name -> numpy array) as ``out_dir/<name>.npy`` ("/" in a name becomes "."), float64 kept, anything
+    else as float32, ``budget`` bytes in all: every array gets an equal share, and one larger than its share is stored as a
+    fixed, seeded sample of its elements (flattened, the same indices on every run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = budget // len(arrays) - 256                      # room for the .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        cap = share // a.itemsize
+        if a.size > cap:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name.replace("/", ".") + ".npy"), a)
 
 
 class ClockSampler:
@@ -184,8 +209,9 @@ def timed_loop(torch, dist, world, device, step_fn, steps, warmup, clocks=None):
     torch.cuda.synchronize(device)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
+    last = None
     for _ in range(steps):
-        step_fn()
+        last = step_fn()
     e1.record()
     torch.cuda.synchronize(device)
     if world > 1:
@@ -196,19 +222,22 @@ def timed_loop(torch, dist, world, device, step_fn, steps, warmup, clocks=None):
         t = torch.tensor([ms], dtype=torch.float64, device=device)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
-    return ms
+    return ms, last
 
 
-def measure(torch, dist, world, device, local, step_dev, step_e2e, steps, warmup, no_e2e, B, n_gpus, h2d, d2h):
-    """Device-timed loop (+ clocks sampled during it) and the end-to-end loop of one arm."""
+def measure(torch, dist, world, device, local, step_dev, step_e2e, steps, warmup, no_e2e, B, n_gpus, h2d, d2h, after_timed=None):
+    """Device-timed loop (+ clocks sampled during it) and the end-to-end loop of one arm.  ``after_timed(last)`` runs between
+    the two with what the last device-timed step returned."""
     clocks = ClockSampler(local)
     clocks.start()
     time.sleep(0.3)
-    ms = timed_loop(torch, dist, world, device, step_dev, steps, warmup, clocks)
+    ms, last = timed_loop(torch, dist, world, device, step_dev, steps, warmup, clocks)
     clk = clocks.stop()
+    if after_timed is not None:
+        after_timed(last)
     e2e = None
     if not no_e2e:
-        ms_e2e = timed_loop(torch, dist, world, device, step_e2e, steps, max(3, warmup // 2))
+        ms_e2e, _ = timed_loop(torch, dist, world, device, step_e2e, steps, max(3, warmup // 2))
         e2e = {"value": B * n_gpus * steps / (ms_e2e / 1e3), "unit": "samples/s", "ms_per_step": ms_e2e / steps,
                "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h}
     return ms, clk, e2e
@@ -383,7 +412,15 @@ def main():
                 eng._graph, eng._bound = None, {}
                 torch.cuda.synchronize(device)
         h2d, d2h = loader.bytes_per_batch, 4
-        ms, clk, e2e = measure(torch, dist, world, device, local, step_dev, step_e2e, args.steps, args.warmup, args.no_e2e, B, n_gpus, h2d, d2h)
+
+        def write_outputs(loss):
+            # what a caller of the step receives (its loss) and the variables it leaves behind, as a checkpoint names them
+            arrays = {"loss": loss.float().cpu().numpy()}
+            arrays.update((k, v.float().numpy()) for k, v in eng.model.reference_state_dict().items())
+            dump_outputs(args.dump_outputs, arrays)
+
+        ms, clk, e2e = measure(torch, dist, world, device, local, step_dev, step_e2e, args.steps, args.warmup, args.no_e2e, B, n_gpus, h2d, d2h,
+                               after_timed=write_outputs if (args.dump_outputs and rank == 0) else None)
         cuda_lstm.check_kernel_errors(device)
         if hasattr(comm, "check_errors"):
             comm.check_errors()
